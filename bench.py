@@ -22,6 +22,7 @@ import json
 import os
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
@@ -157,6 +158,16 @@ def peaks():
     return 6650.0, "fallback (B200_PROFILING.md)"
 
 
+def dump_outputs(path, nav):
+    """--dump-outputs: every field of the nav records the timed path returned for its last step, one <field>.npy per
+    field (float32 fields as they are, the others as float64, exact for the int32 counters), so that two builds run
+    with the same arguments can be compared output for output."""
+    os.makedirs(path, exist_ok=True)
+    for name in nav.dtype.names:
+        a = nav[name]
+        np.save(os.path.join(path, name + ".npy"), np.ascontiguousarray(a, np.float32 if a.dtype == np.float32 else np.float64))
+
+
 def cpu_model():
     try:
         for line in open("/proc/cpuinfo"):
@@ -220,7 +231,7 @@ def bench_reference(args):
         from rebvo_b200 import synth
         seq = synth.Sequence(w=cam["w"], h=cam["h"], seed=seed0, zf=cam["zfx"])
         imu = synth.imu_samples_walk(seq, total, min(IMU_BASE_N, total))
-    info, rec = run_reference("/tmp", ts, base, idx, total, per * args.warmup, gpu_params=params, imu=imu,
+    info, rec = run_reference(tempfile.gettempdir(), ts, base, idx, total, per * args.warmup, gpu_params=params, imu=imu,
                               kc=undistort_of(args.config))
     fps = info["fps"]
     ncpu = os.cpu_count() or 1
@@ -435,10 +446,11 @@ def bench_ours(args):
     if world == 1 and not args.no_cpu_baseline:
         try:
             n = min(620, total)
-            info, rec = run_reference("/tmp", ts, base, idx, n, 20, gpu_params=params, imu=imu, kc=undistort_of(args.config))
+            info, rec = run_reference(tempfile.gettempdir(), ts, base, idx, n, 20, gpu_params=params, imu=imu,
+                                      kc=undistort_of(args.config))
             cpu = {"value": info["fps"], "unit": "frames/s", "cores": 3, "kind": "reference", "cpu_model": cpu_model(),
                    "sample": "first %d frames of the bench stream (20 warm-up) through the unmodified 3-thread REBVO "
-                             "built from /root/reference sources; %d host cpus visible" % (n, os.cpu_count() or 1),
+                             "built from the reference sources; %d host cpus visible" % (n, os.cpu_count() or 1),
                    "mean_dtp0_ms": info["mean_dtp0_ms"], "mean_dtp1_ms": info["mean_dtp1_ms"]}
             from oracle import refapi
             parity = refapi.trajectory_parity(rec, nav_dev)
@@ -477,6 +489,8 @@ def bench_ours(args):
            "e2e_with_mirror": mirror,
            "gpu_launches": int(launches), "gpu_launches_per_frame": launches / (K * B),
            "parity": parity, "roofline": roof, "cpu_baseline": cpu}
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, navs[-1])
     print(json.dumps(out))
     if dist is not None:
         dist.destroy_process_group()
@@ -608,7 +622,7 @@ def bench_config4(args):
             from rebvo_b200 import synth
             n = min(40, total)
             idx = walk_index(total, base_n, 0)
-            path = "/tmp/rebvo_b200_bench4_%d.bin" % os.getpid()
+            path = os.path.join(tempfile.gettempdir(), "rebvo_b200_bench4_%d.bin" % os.getpid())
             synth.write_frames_file(path, ts[:n], base[idx[:n]])
             kv = refapi.ref_params_from(params, Warmup=8)
             if (os.cpu_count() or 1) >= 3:
@@ -639,6 +653,8 @@ def bench_config4(args):
                    "d2h_bytes_per_step": S * B * capi.NAV.itemsize, "ms_per_step": t_e2e_max / K},
            "gpu_launches": int(launches), "gpu_launches_per_frame": launches / frames,
            "parity": parity, "roofline": None, "cpu_baseline": cpu}
+    if args.dump_outputs:   # leading axis: the sequence
+        dump_outputs(args.dump_outputs, np.stack([n[-B:] for n in nav_dev]))
     print(json.dumps(out))
     if dist is not None:
         dist.destroy_process_group()
@@ -654,7 +670,10 @@ def main():
     ap.add_argument("--batch", type=int, default=64)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of this library's pipeline, not of --impl reference")
     if args.impl == "reference":
         bench_reference(args)
     elif args.config == 4:

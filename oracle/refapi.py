@@ -1,8 +1,12 @@
 """TEST INFRASTRUCTURE ONLY: ctypes binding of oracle/_ref/libref_mtrack.so (the unmodified reference
 mtracklib compiled by oracle/build_ref.py).  Only tests/, __graft_entry__.smoke() and bench.py's
 cpu_baseline / reference arm may import this module; the product never does."""
+import atexit
 import ctypes as C
 import os
+import re
+import shutil
+import tempfile
 
 import numpy as np
 
@@ -275,6 +279,35 @@ OUTREC = np.dtype([("t", "f8"), ("Pos", "f8", 3), ("PoseLie", "f8", 3), ("Pose",
                    ("Rot", "f8", 9), ("RKp", "f8"), ("dt", "f8")])
 
 
+# a DT_NEEDED string that names librebvo_b200.so by an absolute path
+_NEEDED_BY_PATH = re.compile(rb"/[^\0]*/librebvo_b200\.so\0")
+_runnable = {}
+
+
+def runnable(exe):
+    """Path to start the oracle program `exe` (oracle/_ref/shim_driver, shim_rebvo) from.  A program linked against a
+    librebvo_b200.so without a soname records the library by the absolute path of the tree it was built in: it does
+    not start once that tree is gone, and would use that tree's library if it were not.  For such a program this
+    returns a copy, under a temporary directory, whose DT_NEEDED entry names the library by file name (the string
+    shrinks in place, NUL-padded) and which sits beside a link to this tree's rebvo_b200/, so that the program's
+    $ORIGIN/../../rebvo_b200 rpath loads this tree's library.  Any other program is returned as it is."""
+    if exe not in _runnable:
+        with open(exe, "rb") as f:
+            data = f.read()
+        _runnable[exe] = exe
+        if _NEEDED_BY_PATH.search(data):
+            d = tempfile.mkdtemp(prefix="rebvo_oracle_")
+            atexit.register(shutil.rmtree, d, True)
+            os.symlink(os.path.join(os.path.dirname(HERE), "rebvo_b200"), os.path.join(d, "rebvo_b200"))
+            os.makedirs(os.path.join(d, "oracle", "_ref"))
+            out = os.path.join(d, "oracle", "_ref", os.path.basename(exe))
+            with open(out, "wb") as f:
+                f.write(_NEEDED_BY_PATH.sub(lambda m: b"librebvo_b200.so".ljust(len(m.group(0)), b"\0"), data))
+            os.chmod(out, 0o755)
+            _runnable[exe] = out
+    return _runnable[exe]
+
+
 def run_full_rebvo(frames_file, out_file, params=None, timeout=600, exe=None):
     """Level B: run the reference's whole 3-thread REBVO on a raw frame file (oracle/ref_driver.cpp).
     exe: another build of the same driver (oracle/_ref/shim_rebvo = the unmodified REBVO sources on the GPU library)."""
@@ -286,7 +319,7 @@ def run_full_rebvo(frames_file, out_file, params=None, timeout=600, exe=None):
         # finite, large stack: the reference keeps O(27*8*K) byte VLAs on thread stacks (SURVEY.md section 7)
         resource.setrlimit(resource.RLIMIT_STACK, (1000000 * 1024, resource.RLIM_INFINITY))
 
-    args = [exe or EXE, frames_file, out_file] + ["%s=%s" % (k, v if isinstance(v, str) else repr(v)) for k, v in (params or {}).items()]
+    args = [runnable(exe or EXE), frames_file, out_file] + ["%s=%s" % (k, v if isinstance(v, str) else repr(v)) for k, v in (params or {}).items()]
     env = dict(os.environ)
     env["LD_LIBRARY_PATH"] = _blas_dir() + ":" + env.get("LD_LIBRARY_PATH", "")
     env.setdefault("OPENBLAS_NUM_THREADS", "1")

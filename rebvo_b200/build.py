@@ -42,7 +42,9 @@ def build(force=False, verbose=False):
 
     with ThreadPoolExecutor(max_workers=len(SOURCES)) as ex:
         objs = list(ex.map(cc, SOURCES))
-    cmd = [NVCC, "-shared", "-o", LIB] + objs + ["-lcudart"]
+    # the soname makes programs linked against this file record "librebvo_b200.so" rather than its absolute build path,
+    # so that they find it through their rpath wherever the tree is moved to
+    cmd = [NVCC, "-shared", "-Xlinker", "-soname=librebvo_b200.so", "-o", LIB] + objs + ["-lcudart"]
     r = subprocess.run(cmd, capture_output=True, text=True)
     if r.returncode != 0:
         raise RuntimeError("link failed:\n" + r.stdout + r.stderr)

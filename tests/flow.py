@@ -103,6 +103,44 @@ KL_FIELDS = ["p_inx", "m_m", "u_m", "n_m", "c_p", "rho", "s_rho", "rho_nr", "s_r
              "p_m_0", "m_id", "m_id_f", "m_id_kf", "m_num", "p_id", "n_id"]
 
 
+# keyline arrays of the later stages and the array each one was derived from (parents first)
+KL_PARENT = {"rot_kl": "f0_kl", "fm_kl": "f1_kl", "dm_kl": "fm_kl", "reg_kl": "dm_kl", "ekf_kl": "reg_kl"}
+
+
+def save_golden(path, arrays):
+    """np.savez layout with LZMA members (np.load reads it).  A keyline array of KL_PARENT is stored as only the fields
+    that differ from its parent's, under "<name>.<field>": together this keeps the file under 1 MB."""
+    import io
+    import zipfile
+    with zipfile.ZipFile(path, "w", zipfile.ZIP_LZMA) as zf:
+        def put(name, a):
+            buf = io.BytesIO()
+            np.save(buf, np.ascontiguousarray(a))
+            zf.writestr(name + ".npy", buf.getvalue())
+        for k, a in arrays.items():
+            if k not in KL_PARENT:
+                put(k, a)
+                continue
+            parent = arrays[KL_PARENT[k]]
+            assert len(parent) == len(a), k
+            for f in a.dtype.names:
+                if a[f].tobytes() != parent[f].tobytes():
+                    put("%s.%s" % (k, f), a[f])
+
+
+def load_golden(path):
+    """The arrays save_golden wrote, keyline arrays of KL_PARENT rebuilt whole."""
+    z = np.load(path)
+    out = {k: z[k] for k in z.files if "." not in k}
+    for k, parent in KL_PARENT.items():
+        a = out[parent].copy()
+        for f in a.dtype.names:
+            if "%s.%s" % (k, f) in z.files:
+                a[f] = z["%s.%s" % (k, f)]
+        out[k] = a
+    return out
+
+
 def compare(ref, got, tol_keys=(), rtol=1e-9, loose=()):
     """Bitwise comparison of two flow outputs except for keys starting with a prefix in tol_keys.  Returns a list
     of failure strings."""

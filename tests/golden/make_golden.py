@@ -13,14 +13,14 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, os.path.dirname(HERE))
 sys.path.insert(0, os.path.dirname(os.path.dirname(HERE)))
 
-from flow import SMALL, run_flow, run_imu_rows, small_frames  # noqa: E402
+from flow import SMALL, run_flow, run_imu_rows, save_golden, small_frames  # noqa: E402
 from oracle import build_ref, refapi  # noqa: E402
 
 if __name__ == "__main__":
     assert build_ref.build(level_b=False), "reference sources not available"
     f0, f1 = small_frames()
     out = run_flow(refapi.RefMap, SMALL, f0, f1, refapi.so3_exp)
-    np.savez_compressed(os.path.join(HERE, "flow_small.npz"), f0=f0, f1=f1, **out)
+    save_golden(os.path.join(HERE, "flow_small.npz"), dict(f0=f0, f1=f1, **out))
     print("wrote flow_small.npz:", {k: (v.shape, str(v.dtype)[:12]) for k, v in list(out.items())[:6]}, "...")
     print("kn:", out["f0_kn_tresh"], out["f1_kn_tresh"], "dm:", out["dm_count"], "min V:", out["min_V"])
     imu = run_imu_rows(refapi.RefMap, refapi, SMALL, f0, f1)

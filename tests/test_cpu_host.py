@@ -142,8 +142,9 @@ def test_shim_imu_mirrors_compile():
     replay driver does not instantiate: compile them against the reference's own TooN / cam_model headers."""
     import shutil
     import subprocess
+    from oracle import build_ref
     repo = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    ref = "/root/reference"
+    ref = build_ref.REF
     out = os.path.join(repo, "oracle", "_ref")
     if not os.path.isdir(ref) or not os.path.isdir(os.path.join(out, "toon")) or shutil.which("g++") is None:
         pytest.skip("reference headers not available here")

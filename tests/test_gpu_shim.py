@@ -22,7 +22,7 @@ def test_shim_classes_reproduce_reference_flow(built, tmp_path):
     ts, fr = seq.frames(NF)
     path = str(tmp_path / "frames.bin")
     synth.write_frames_file(path, ts, fr)
-    r = subprocess.run([exe, path, path + ".shim"], capture_output=True, text=True, timeout=600)
+    r = subprocess.run([refapi.runnable(exe), path, path + ".shim"], capture_output=True, text=True, timeout=600)
     assert r.returncode == 0, r.stderr[-2000:]
     with open(path + ".shim", "rb") as f:
         n, sz = np.frombuffer(f.read(8), np.int32)

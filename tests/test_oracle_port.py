@@ -10,7 +10,7 @@ import pytest
 
 import ctypes as C
 
-from flow import DOG_THRESH, PLANE_FIT, POS_NEG, SMALL, compare, run_flow, run_imu_rows, small_frames
+from flow import DOG_THRESH, PLANE_FIT, POS_NEG, SMALL, compare, load_golden, run_flow, run_imu_rows, small_frames
 
 GOLD = os.path.join(os.path.dirname(__file__), "golden", "flow_small.npz")
 TOL = ("min_V", "min_W", "min_RVel", "min_RW0", "min_W_X", "min_scalars")
@@ -18,8 +18,7 @@ TOL = ("min_V", "min_W", "min_RVel", "min_RW0", "min_W_X", "min_scalars")
 
 @pytest.fixture(scope="module")
 def golden():
-    z = np.load(GOLD)
-    return {k: z[k] for k in z.files}
+    return load_golden(GOLD)
 
 
 def _override(g):

@@ -1,5 +1,6 @@
+import os
 import sys
-sys.path.insert(0, '/root/repo')
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np
 from rebvo_b200 import capi, synth
 cam = synth.EUROC
